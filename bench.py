@@ -39,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 
 def _baseline_metric():
@@ -226,8 +227,10 @@ def run_reference_arm(args):
         impl.infer(model, images[:n], threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        impl.infer(model, images[:n], threads=threads)
+        logits, labels = impl.infer(model, images[:n], threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": logits, "labels": labels})
     value = n * args.steps / dt
     base["value"] = value
     base["sample"] = f"each step = {n} of the {args.batch} synthetic images; " + base["sample"].split(", best of")[1].split(", ", 1)[1]
@@ -240,6 +243,27 @@ def run_reference_arm(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }), file=RESULT_OUT, flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write each array (all with the same leading row count) as out_dir/<name>.npy: float32, or float64 where float32 would not
+    hold its integers exactly.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of rows is written instead, with the
+    indices of those rows as out_dir/rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    exact32 = lambda a: a.size == 0 or (-(1 << 24) <= a.min() and a.max() <= (1 << 24))
+    arrays = {k: a.astype(np.float32 if exact32(a) else np.float64) for k, a in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a.nbytes // max(n, 1) for a in arrays.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(seed).choice(n, size=keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def workload_name(name, model, batch):
@@ -594,7 +618,11 @@ def main():
     ap.add_argument("--sustain-seconds", type=float, default=1.0)
     ap.add_argument("--path", default="auto", choices=["auto", "layers", "tcgen05"])
     ap.add_argument("--dist", default="uniform", choices=["uniform", "mnist"], help="synthetic image distribution (SURVEY.md 8d config 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the logits and labels of the last timed step as DIR/<name>.npy (rank 0; "
+                    "inputs are seeded, so runs with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -762,6 +790,9 @@ def main():
             latency = latency_batch1(args.model)
 
     if rank == 0:
+        if args.dump_outputs:
+            last_logits, last_labels = snap_plain[(args.steps - 1) & 1]   # DeviceBatch alternates its two buffers per step
+            dump_outputs(args.dump_outputs, {"logits": last_logits, "labels": last_labels})
         out = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

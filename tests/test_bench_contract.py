@@ -23,6 +23,36 @@ def test_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1 and d["gpu_launches"] == 0
 
 
+def test_reference_arm_dumps_the_last_step(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--batch", "4096", "--steps", "2",
+                          "--warmup", "3", "--dump-outputs", str(tmp_path)], cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stderr[-2000:]
+    n = json.loads(out.stdout)["config"]["sample_per_step"]
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle.oracle import Oracle
+    want_logits, want_labels = Oracle().infer(bench.load_model("fc"), bench.synth_images(4096, 256, 1234)[:n])
+    logits, labels = np.load(tmp_path / "logits.npy"), np.load(tmp_path / "labels.npy")
+    assert logits.dtype == labels.dtype == np.float32 and sorted(os.listdir(tmp_path)) == ["labels.npy", "logits.npy"]
+    assert np.array_equal(logits, want_logits) and np.array_equal(labels, want_labels)
+
+
+def test_dump_outputs_samples_rows_above_the_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1000)
+    logits = np.arange(4000, dtype=np.int32).reshape(400, 10) * 5000        # beyond 2**24: float64
+    labels = np.arange(400, dtype=np.uint32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"logits": logits, "labels": labels})
+    got = {f: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert sorted(got) == ["labels.npy", "logits.npy", "rows.npy"] and sum(a.nbytes for a in got.values()) <= 1000
+    rows = got["rows.npy"].astype(np.int64)
+    assert got["logits.npy"].dtype == np.float64 and np.array_equal(got["logits.npy"], logits[rows])
+    assert got["labels.npy"].dtype == np.float32 and np.array_equal(got["labels.npy"], labels[rows])
+    assert np.array_equal(np.load(tmp_path / "b" / "rows.npy"), got["rows.npy"])   # the same sample every time
+
+
 def test_reference_arm_other_ranks_stay_silent():
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--batch", "4096",

@@ -1,6 +1,6 @@
 """Pin the oracle (oracle/bitnet_oracle.c) against the reference: golden vectors made by the unmodified
-reference kernels (tests/golden/make_golden.py), the reference's own label KAT, and -- when oracle/_ref is
-present -- exhaustive decode sweeps and random function-level comparisons against the reference itself."""
+reference kernels (tests/golden/make_golden.py), the reference's own label KAT, exhaustive decode sweeps, and
+random function-level comparisons against the reference's outputs stored by tests/golden/make_reference_vectors.py."""
 import json
 import os
 import zlib
@@ -98,10 +98,16 @@ def test_ternary_all_words(oracle):
     assert np.array_equal(oracle.decode_fc(packed, M.ENC_TERNARY, 10, 59049), trits)
 
 
-# ---- direct comparisons with the unmodified reference (skipped where oracle/_ref is absent) -------------
+# ---- comparisons with the unmodified reference kernels: their outputs on these seeded inputs are stored in
+# golden/reference_vectors.npz (written by golden/make_reference_vectors.py, which calls the same *_cases generators) ---
 
-@pytest.mark.parametrize("enc", [1, 2, 4, 12, 16, 20, 36, 64, 3])
-def test_fclayer_vs_reference(oracle, reference, enc):
+FCLAYER_ENCODINGS = [1, 2, 4, 12, 16, 20, 36, 64, 3]
+WHOLE_MODELS = ["fc", "cnn", "cnn_48", "binary160", "ternary64", "rand_fp130_64", "rand_nf4_64", "1k"]
+LOGITS_HEAD = 80   # rows stored in full per model: the MNIST-like, all -128, all 127 and all-zero images
+
+
+def fclayer_cases(enc):
+    """(n_in, n_out, activations, weights) of one fully connected layer per shape."""
     rng = np.random.default_rng(enc)
     for n_in, n_out in [(256, 64), (64, 10), (160, 160), (320, 7)]:
         if enc == 64:
@@ -110,10 +116,10 @@ def test_fclayer_vs_reference(oracle, reference, enc):
         else:
             w = rng.integers(0, 2 ** 32, size=n_out * n_in // 4 + 4, dtype=np.uint64).astype(np.uint32)
         act = rng.integers(-128, 128, size=n_in + 16).astype(np.int8)
-        assert np.array_equal(oracle.fclayer(act, w, enc, n_in, n_out), reference.fclayer(act, w, enc, n_in, n_out))
+        yield n_in, n_out, act, w
 
 
-def test_relunorm_vs_reference(oracle, reference):
+def relunorm_cases():
     rng = np.random.default_rng(7)
     for trial in range(300):
         n = int(rng.integers(1, 300))
@@ -123,25 +129,20 @@ def test_relunorm_vs_reference(oracle, reference):
             x = -np.abs(x) - 1
         if trial % 11 == 0:
             x[rng.integers(0, n)] = 2 ** (7 + trial % 20) - 1
-        a, pa = oracle.relunorm(x)
-        b, pb = reference.relunorm(x)
-        assert pa == pb and np.array_equal(a, b)
+        yield x
 
 
-def test_conv_pool_vs_reference(oracle, reference):
+def conv_pool_cases():
+    """(xy, activations, 3x3 weights), twenty per image size."""
     rng = np.random.default_rng(9)
     for xy in (16, 14, 6, 4, 3):
         for _ in range(20):
             act = rng.integers(-20000, 20000, size=xy * xy).astype(np.int32)
             w = rng.integers(-128, 128, size=9).astype(np.int8)
-            assert np.array_equal(oracle.conv33relu(act, w, xy, 4), reference.conv33relu(act, w, xy, 4))
-            if xy % 2 == 0:
-                assert np.array_equal(oracle.maxpool22(act, xy), reference.maxpool22(act, xy))
+            yield xy, act, w
 
 
-@pytest.mark.parametrize("name", ["fc", "cnn", "cnn_48", "binary160", "ternary64", "rand_fp130_64", "rand_nf4_64", "1k"])
-def test_whole_model_vs_reference_random(oracle, reference, name):
-    m = load_model(name)
+def whole_model_images(m):
     rng = np.random.default_rng(11)
     n = 3000 if m.model_class == M.MODEL_FCMNIST else 600
     imgs = rng.integers(-128, 128, size=(n, 256)).astype(np.int8)
@@ -149,6 +150,44 @@ def test_whole_model_vs_reference_random(oracle, reference, name):
     imgs[50:60] = -128
     imgs[60:70] = 127
     imgs[70:80] = 0
-    lo, la = oracle.infer(m, imgs)
-    lr, lar = reference.infer(m, imgs)
-    assert np.array_equal(lo, lr) and np.array_equal(la, lar)
+    return imgs
+
+
+def logits_crc32(logits):
+    return zlib.crc32(np.ascontiguousarray(logits, dtype="<i4").tobytes())
+
+
+@pytest.mark.parametrize("enc", FCLAYER_ENCODINGS)
+def test_fclayer_vs_reference(oracle, reference_vectors, enc):
+    for n_in, n_out, act, w in fclayer_cases(enc):
+        want = reference_vectors[f"fclayer/{enc}/{n_in}x{n_out}"]
+        assert np.array_equal(oracle.fclayer(act, w, enc, n_in, n_out), want), (n_in, n_out)
+
+
+def test_relunorm_vs_reference(oracle, reference_vectors):
+    want_out, want_pos = reference_vectors["relunorm/out"], reference_vectors["relunorm/pos"]
+    at = 0
+    for trial, x in enumerate(relunorm_cases()):
+        a, pa = oracle.relunorm(x)
+        assert pa == want_pos[trial] and np.array_equal(a, want_out[at:at + x.size]), trial
+        at += x.size
+    assert at == want_out.size
+
+
+def test_conv_pool_vs_reference(oracle, reference_vectors):
+    seen = {}
+    for xy, act, w in conv_pool_cases():
+        k = seen[xy] = seen.get(xy, -1) + 1
+        assert np.array_equal(oracle.conv33relu(act, w, xy, 4), reference_vectors[f"conv/{xy}"][k]), (xy, k)
+        if xy % 2 == 0:
+            assert np.array_equal(oracle.maxpool22(act, xy), reference_vectors[f"pool/{xy}"][k]), (xy, k)
+
+
+@pytest.mark.parametrize("name", WHOLE_MODELS)
+def test_whole_model_vs_reference_random(oracle, reference_vectors, name):
+    """Labels of every image and logits of the first LOGITS_HEAD are stored; the full logits array by its CRC-32."""
+    m = load_model(name)
+    lo, la = oracle.infer(m, whole_model_images(m))
+    assert np.array_equal(lo[:LOGITS_HEAD], reference_vectors[f"model/{name}/logits_head"])
+    assert logits_crc32(lo) == int(reference_vectors[f"model/{name}/logits_crc32"])
+    assert np.array_equal(la, reference_vectors[f"model/{name}/labels"])

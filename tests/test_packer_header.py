@@ -1,14 +1,14 @@
 """Host logic either side of the path: the BitNetMCU_model.h parser, the exportquant-compatible packer, the BNM1 blob."""
+import json
 import os
+import zlib
 
 import numpy as np
 import pytest
 
-from conftest import load_model, model_names
+from conftest import GOLDEN, load_model, model_names
 from bitnetmcu_b200 import model as M
 from bitnetmcu_b200 import pack as P
-
-REF = "/root/reference"
 
 
 @pytest.mark.parametrize("enc", [M.ENC_BINARY, M.ENC_2BITSYM, M.ENC_4BITSYM, M.ENC_4BIT, M.ENC_8BIT, M.ENC_FP130, M.ENC_NF4])
@@ -101,17 +101,36 @@ def test_blob_roundtrip(name):
             assert a.weights.dtype == b.weights.dtype and np.array_equal(a.weights, b.weights)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs /root/reference")
-def test_parser_on_every_shipped_reference_header():
-    import glob
-    heads = [os.path.join(REF, "BitNetMCU_model_fc.h"), os.path.join(REF, "BitNetMCU_model_cnn.h")] + \
-        sorted(glob.glob(os.path.join(REF, "mcu", "BitNetMCU_model_*.h")))
-    assert len(heads) == 11
-    for h in heads:
-        m = M.parse_header(h)
+def header_fingerprint(m):
+    """What a header parse yields, in JSON form: class, MACs per image, and per layer its shape and the CRC-32 of its weights."""
+    return {"model_class": m.model_class, "macs_per_image": m.macs_per_image,
+            "layers": [[l.name, l.kind, l.bitperweight, l.n_in, l.n_out, l.in_channels, l.groups,
+                        None if l.weights is None else zlib.crc32(np.ascontiguousarray(l.weights).tobytes())] for l in m.layers]}
+
+
+def test_parser_on_every_shipped_reference_header(tmp_path):
+    """The reference ships eleven model headers (ten distinct models: the CNN one twice) and a test-data header.
+    golden/shipped_headers.json records what the parser read from each model header
+    (tests/golden/make_reference_vectors.py): every fixture model is exactly that parse, and so is the parse of the header
+    written for it.  The test digits, written in the test-data header's hex layout, parse back unchanged."""
+    shipped = json.load(open(os.path.join(GOLDEN, "shipped_headers.json")))
+    assert len(shipped) == 11
+    for header, want in shipped.items():
+        m = load_model(want["fixture"])
+        assert header_fingerprint(m) == want["parsed"], header
         assert m.fc_layers and m.macs_per_image > 0
-    imgs, labels = M.parse_test_data_header(os.path.join(REF, "BitNetMCU_MNIST_test_data.h"))
+        path = os.path.join(tmp_path, os.path.basename(header))
+        P.write_header(m, path)
+        assert header_fingerprint(M.parse_header(path)) == want["parsed"], header
+    d = np.load(os.path.join(GOLDEN, "digits.npz"))
+    path = os.path.join(tmp_path, "BitNetMCU_MNIST_test_data.h")
+    with open(path, "w") as f:
+        for i, (img, label) in enumerate(zip(d["images"], d["labels"])):
+            rows = [", ".join("0x%02X" % v for v in img[r:r + 16].view(np.uint8)) for r in range(0, 256, 16)]
+            f.write(f"int8_t input_data_{i}[256] = {{\n" + ",\n".join(rows) + "\n};\n" + f"uint8_t label_{i} = {int(label)};\n")
+    imgs, labels = M.parse_test_data_header(path)
     assert imgs.shape == (10, 256) and labels.tolist() == [3, 2, 0, 9, 0, 6, 9, 2, 7, 7] and imgs[0, 0] == -20   # 0xEC narrowed to int8
+    assert np.array_equal(imgs, d["images"])
 
 
 def test_blob_roundtrip_names_layers_like_the_reference_harness():
