@@ -21,6 +21,7 @@ EXPORTED = [
     "bnm_quantize_images", "bnm_quantize_images_device",
     "bnm_infer_batch_device_gather", "bnm_device_alloc", "bnm_device_free", "bnm_ipc_export", "bnm_ipc_open", "bnm_ipc_close",
     "bnm_enable_peer_access", "bnm_emulate_inference_quantized", "bnm_infer_batch_device_f32",
+    "bnm_model_n_taps", "bnm_model_tap_width", "bnm_model_tap_stride", "bnm_infer_batch_device_taps", "bnm_infer_batch_taps",
 ]
 
 PATH_AUTO, PATH_LAYERS, PATH_TCGEN05 = 0, 1, 2
@@ -40,6 +41,14 @@ class BnmGather(C.Structure):
     """bnm_gather (include/bitnetmcu_b200.h): destinations of the fused result exchange."""
     _fields_ = [("n_labels_dst", C.c_uint32), ("n_logits_dst", C.c_uint32), ("labels_dst", C.c_void_p * MAX_GATHER_DST),
                 ("logits_dst", C.c_void_p * MAX_GATHER_DST), ("row_offset", C.c_size_t), ("labels_u8", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+MAX_TAPS = 8
+
+
+class BnmTaps(C.Structure):
+    """bnm_taps (include/bitnetmcu_b200.h): per tap an int8 [n][stride] buffer, or NULL when the tap is not wanted."""
+    _fields_ = [("act", C.c_void_p * MAX_TAPS)]
 
 
 _lib = None
@@ -79,6 +88,9 @@ def load() -> C.CDLL:
         "bnm_enable_peer_access": (C.c_int, [C.c_int, C.c_int]),
         "bnm_emulate_inference_quantized": (C.c_int, [vp, vp, sz, vp]),
         "bnm_infer_batch_device_f32": (C.c_int, [vp, vp, sz, vp, vp, vp]),
+        "bnm_model_n_taps": (u32, [vp]), "bnm_model_tap_width": (u32, [vp, u32]), "bnm_model_tap_stride": (u32, [vp, u32]),
+        "bnm_infer_batch_device_taps": (C.c_int, [vp, vp, sz, vp, vp, C.POINTER(BnmTaps), vp]),
+        "bnm_infer_batch_taps": (C.c_int, [vp, vp, sz, vp, vp, C.POINTER(BnmTaps)]),
         "ReLUNorm": (u32, [vp, vp, u32]),
         "processfclayer": (None, [vp, vp, i32, u32, u32, vp]),
         "processconv33ReLU": (vp, [vp, vp, u32, u32, vp]),

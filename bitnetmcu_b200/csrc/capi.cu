@@ -389,8 +389,10 @@ extern "C" int64_t bnm_model_get_option(const bnm_model *m, int option) {
 static const size_t kLayeredChunk = 1 << 17;   // images per pass of the layer-by-layer path (bounds its scratch)
 static const size_t kFusedCnnChunk = 1 << 20;  // fused path, CNN models: images per front-end + FC launch pair (256 B of features each)
 
-// FC chain, one CUDA-core kernel per layer: input int8 [n][in_stride]
-static int run_fc_layers(bnm_model *m, const int8_t *in, uint32_t in_stride, size_t n, int32_t *logits, uint32_t *labels, cudaStream_t st) {
+// FC chain, one CUDA-core kernel per layer: input int8 [n][in_stride].  taps (may be null): a requested hidden row is written
+// straight into its tap buffer (at the next layer's k_pad, the stride the next layer reads) instead of the ping-pong scratch.
+static int run_fc_layers(bnm_model *m, const int8_t *in, uint32_t in_stride, size_t n, int32_t *logits, uint32_t *labels, cudaStream_t st,
+                         const FcTaps *taps = nullptr) {
     const int8_t *act = in;
     uint32_t stride = in_stride;
     const size_t nl = m->fc.size();
@@ -402,7 +404,7 @@ static int run_fc_layers(bnm_model *m, const int8_t *in, uint32_t in_stride, siz
         if (last) {
             if (labels) launch_relunorm(acc, m->fc[l].n_out, nullptr, 0, labels, n, st);
         } else {
-            int8_t *next = m->d_act[l & 1];
+            int8_t *next = taps && taps->act[l] ? taps->act[l] : m->d_act[l & 1];
             uint32_t next_stride = m->fc[l + 1].k_pad;
             launch_relunorm(acc, m->fc[l].n_out, next, next_stride, nullptr, n, st);
             act = next;
@@ -433,9 +435,16 @@ extern "C" int bnm_infer_launch_count(const bnm_model *m, size_t n) {
     return (int)(chunks * per);
 }
 
+static uint32_t n_taps(const bnm_model *m) { return (uint32_t)m->fc.size() - 1 + (m->model_class == BNM_MODEL_CNNMNIST ? 1 : 0); }
+static uint32_t tap_stride(const bnm_model *m, uint32_t t) {
+    const uint32_t t0 = m->model_class == BNM_MODEL_CNNMNIST ? 1 : 0;
+    return t < t0 ? m->feat_stride : m->fc[t - t0 + 1].k_pad;
+}
+
 // slot_feat: a caller-owned feature buffer for n images (the host pipeline's per-slot buffers); null = the model's own scratch
+// taps: checked by check_taps, at least one entry set (null: none)
 static int infer_device_impl(bnm_model *m, const int8_t *images, size_t n, int32_t *logits, uint32_t *labels, const GatherDst *gather, void *stream,
-                             int8_t *slot_feat = nullptr) {
+                             int8_t *slot_feat = nullptr, const bnm_taps *taps = nullptr) {
     if (!m || (n && (!images || !logits))) return fail(BNM_E_ARG, "bnm_infer_batch_device: null argument");
     if (n == 0) return 0;
     if ((uintptr_t)images & 15) return fail(BNM_E_ARG, "the device image buffer must be 16-byte aligned (TMA)");
@@ -445,8 +454,20 @@ static int infer_device_impl(bnm_model *m, const int8_t *images, size_t n, int32
     const bool fused = bnm_model_active_path(m) == BNM_PATH_TCGEN05;
     const bool cnn = m->model_class == BNM_MODEL_CNNMNIST;
     if (gather && !fused) return fail(BNM_E_UNSUPPORTED, "the fused result exchange needs the tcgen05 path (model: %s)", m->plan_err.c_str());
+    if (gather && taps) return fail(BNM_E_UNSUPPORTED, "activation taps are not available with the fused result exchange");
+    const uint32_t t0 = cnn ? 1 : 0;   // FC layer l's row is tap t0 + l
+    // FC taps of the images from row b on
+    auto fc_taps_at = [&](size_t b, FcTaps &ft) -> const FcTaps * {
+        if (!taps) return nullptr;
+        for (size_t l = 0; l < (size_t)kMaxFcLayers; l++) {
+            const uint32_t t = t0 + (uint32_t)l;
+            ft.act[l] = l + 1 < m->fc.size() && taps->act[t] ? taps->act[t] + b * tap_stride(m, t) : nullptr;
+        }
+        return &ft;
+    };
+    FcTaps ft;
     if (fused && !cnn) {
-        int rc = fc_chain_launch(m->plan, images, n, logits, labels, gather, st);
+        int rc = fc_chain_launch(m->plan, images, n, logits, labels, gather, st, fc_taps_at(0, ft));
         return rc ? fail(BNM_E_CUDA, "fused FC kernel launch failed (%d): %s", rc, cudaGetErrorString(cudaGetLastError())) : 0;
     }
     const size_t chunk = slot_feat ? n : std::min(n, fused ? kFusedCnnChunk : kLayeredChunk);
@@ -461,18 +482,20 @@ static int infer_device_impl(bnm_model *m, const int8_t *images, size_t n, int32
         const int8_t *fc_in = img;
         uint32_t fc_stride = m->img_bytes;
         if (cnn) {
-            rc = run_cnn_front(m, img, nb, feat, st);
+            // tap 0 requested: the front-end writes the features straight into it and the FC chain reads them from there
+            int8_t *f = taps && taps->act[0] ? taps->act[0] + b * m->feat_stride : feat;
+            rc = run_cnn_front(m, img, nb, f, st);
             if (rc) return rc;
-            fc_in = feat;
+            fc_in = f;
             fc_stride = m->feat_stride;
         }
         if (fused) {
             GatherDst gchunk;
             if (gather) { gchunk = *gather; gchunk.row_offset += b; }
-            rc = fc_chain_launch(m->plan, fc_in, nb, lg, lb, gather ? &gchunk : nullptr, st);
+            rc = fc_chain_launch(m->plan, fc_in, nb, lg, lb, gather ? &gchunk : nullptr, st, fc_taps_at(b, ft));
             if (rc) return fail(BNM_E_CUDA, "fused FC kernel launch failed (%d)", rc);
         } else {
-            rc = run_fc_layers(m, fc_in, fc_stride, nb, lg, lb, st);
+            rc = run_fc_layers(m, fc_in, fc_stride, nb, lg, lb, st, fc_taps_at(b, ft));
             if (rc) return rc;
         }
     }
@@ -493,6 +516,88 @@ extern "C" int bnm_infer_batch_device_gather(bnm_model *m, const int8_t *images,
         for (uint32_t d = 0; d < gather->n_logits_dst; d++)
             if ((uintptr_t)gather->logits_dst[d] & 7) return fail(BNM_E_ARG, "gather logits buffers must be 8-byte aligned");
     return infer_device_impl(m, images, n, logits, labels, reinterpret_cast<const GatherDst *>(gather), stream);
+}
+
+// -----------------------------------------------------------------------------------------------
+// activation taps (section 7 of the header)
+// -----------------------------------------------------------------------------------------------
+struct DevBuf {
+    void *p = nullptr;
+    ~DevBuf() { if (p) cudaFree(p); }
+    int alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 16) == cudaSuccess ? 0 : -1; }
+    template <class T> T *as() { return static_cast<T *>(p); }
+};
+
+extern "C" uint32_t bnm_model_n_taps(const bnm_model *m) { return m ? n_taps(m) : 0; }
+extern "C" uint32_t bnm_model_tap_width(const bnm_model *m, uint32_t t) {
+    if (!m || t >= n_taps(m)) return 0;
+    const uint32_t t0 = m->model_class == BNM_MODEL_CNNMNIST ? 1 : 0;
+    return t < t0 ? m->channels * 4 : m->fc[t - t0].n_out;
+}
+extern "C" uint32_t bnm_model_tap_stride(const bnm_model *m, uint32_t t) { return m && t < n_taps(m) ? tap_stride(m, t) : 0; }
+
+// 0: taps usable for this call; *any = some entry is set
+static int check_taps(const bnm_model *m, const bnm_taps *taps, bool device, bool *any) {
+    *any = false;
+    if (!taps) return 0;
+    const uint32_t nt = n_taps(m);
+    for (uint32_t t = 0; t < BNM_MAX_TAPS; t++) {
+        if (!taps->act[t]) continue;
+        if (t >= nt) return fail(BNM_E_ARG, "tap %u requested, the model has %u taps", t, nt);
+        if (device && ((uintptr_t)taps->act[t] & 15)) return fail(BNM_E_ARG, "tap %u: the device buffer must be 16-byte aligned", t);
+        *any = true;
+    }
+    // the fused kernel stores a hidden row n_pad = round_up(n_out, 16) bytes wide: it has to fit the stride the next layer reads
+    const uint32_t t0 = m->model_class == BNM_MODEL_CNNMNIST ? 1 : 0;
+    for (uint32_t t = t0; *any && t < nt; t++)
+        if (taps->act[t] && m->fc[t - t0].n_pad > tap_stride(m, t))
+            return fail(BNM_E_UNSUPPORTED, "tap %u: FC layer %u has %u outputs, the next layer reads %u", t, t - t0, m->fc[t - t0].n_out,
+                        m->fc[t - t0 + 1].n_in);
+    return 0;
+}
+
+extern "C" int bnm_infer_batch_device_taps(bnm_model *m, const int8_t *images, size_t n, int32_t *logits, uint32_t *labels,
+                                           const bnm_taps *taps, void *stream) {
+    static_assert(BNM_MAX_TAPS == kMaxFcLayers, "a CNN model with 8 FC layers has 8 taps");
+    if (!m) return fail(BNM_E_ARG, "bnm_infer_batch_device_taps: null model");
+    bool any = false;
+    if (int rc = check_taps(m, taps, true, &any)) return rc;
+    return infer_device_impl(m, images, n, logits, labels, nullptr, stream, nullptr, any ? taps : nullptr);
+}
+
+extern "C" int bnm_infer_batch_taps(bnm_model *m, const int8_t *images, size_t n, int32_t *logits, uint32_t *labels, const bnm_taps *taps) {
+    if (!m) return fail(BNM_E_ARG, "bnm_infer_batch_taps: null model");
+    bool any = false;
+    if (int rc = check_taps(m, taps, false, &any)) return rc;
+    if (!any) return bnm_infer_batch(m, images, n, logits, labels);
+    if (n && (!images || !logits)) return fail(BNM_E_ARG, "bnm_infer_batch_taps: null argument");
+    if (n == 0) return 0;
+    CU_TRY(cudaSetDevice(m->device));
+    const size_t chunk = std::min(n, m->chunk_images);
+    const uint32_t nt = n_taps(m);
+    DevBuf d_img, d_log, d_lab, d_tap[BNM_MAX_TAPS];
+    bnm_taps dt{};
+    if (d_img.alloc(chunk * m->img_bytes) || d_log.alloc(chunk * m->n_classes * sizeof(int32_t)) || d_lab.alloc(chunk * sizeof(uint32_t)))
+        return fail(BNM_E_CUDA, "cudaMalloc failed");
+    for (uint32_t t = 0; t < nt; t++) {
+        if (!taps->act[t]) continue;
+        if (d_tap[t].alloc(chunk * tap_stride(m, t))) return fail(BNM_E_CUDA, "cudaMalloc failed");
+        dt.act[t] = d_tap[t].as<int8_t>();
+    }
+    cudaStream_t st = m->slots[0].stream;
+    for (size_t b = 0; b < n; b += chunk) {
+        const size_t nb = std::min(chunk, n - b);
+        CU_TRY(cudaMemcpyAsync(d_img.p, images + b * m->img_bytes, nb * m->img_bytes, cudaMemcpyHostToDevice, st));
+        int rc = infer_device_impl(m, d_img.as<int8_t>(), nb, d_log.as<int32_t>(), labels ? d_lab.as<uint32_t>() : nullptr, nullptr, st, nullptr, &dt);
+        if (rc) { cudaStreamSynchronize(st); return rc; }
+        CU_TRY(cudaMemcpyAsync(logits + b * m->n_classes, d_log.p, nb * m->n_classes * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        if (labels) CU_TRY(cudaMemcpyAsync(labels + b, d_lab.p, nb * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        for (uint32_t t = 0; t < nt; t++)
+            if (dt.act[t])
+                CU_TRY(cudaMemcpyAsync(taps->act[t] + b * tap_stride(m, t), dt.act[t], nb * tap_stride(m, t), cudaMemcpyDeviceToHost, st));
+    }
+    CU_TRY(cudaStreamSynchronize(st));
+    return 0;
 }
 
 // -----------------------------------------------------------------------------------------------
@@ -624,13 +729,6 @@ extern "C" void bnm_host_free(void *p) { if (p) cudaFreeHost(p); }
 // -----------------------------------------------------------------------------------------------
 // the four kernels, batched over host buffers
 // -----------------------------------------------------------------------------------------------
-struct DevBuf {
-    void *p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    int alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 16) == cudaSuccess ? 0 : -1; }
-    template <class T> T *as() { return static_cast<T *>(p); }
-};
-
 static int require_device() {
     if (bnm_device_count() == 0) return fail(BNM_E_NODEV, "no CUDA device: this engine has no CPU fallback");
     return 0;

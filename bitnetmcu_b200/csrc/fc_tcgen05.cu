@@ -72,6 +72,10 @@ struct ChainParams {
     uint32_t in_elems;                // real elements per image row (<= 256 for the float path)
     uint32_t off_fring;               // float-input launches: smem offset of the quantiser warps' float rings (8 warps x 2 slots x 4 kB)
     uint32_t off_gstage;              // gather launches: smem offset of the per-warp staging rows for the bulk peer stores (0: none)
+    // activation taps (fc_chain_kernel<..., kTaps>): hidden layer l's int8 ReLUNorm row of image i is also stored at
+    // tap[l] + i * tap_stride[l] (null: not wanted).  The stride is the next layer's k_pad, set at plan creation.
+    int8_t *tap[kMaxFcLayers];
+    uint32_t tap_stride[kMaxFcLayers];
 };
 
 struct FcChainPlan {
@@ -161,8 +165,16 @@ __device__ __forceinline__ int max16(const uint32_t (&v)[16], int m) {
     return max(m, m2);
 }
 
-// hidden-layer epilogue, the common 64-wide case: one TMEM load of the whole row, one TMEM store of the 16 packed words
-__device__ __forceinline__ void relunorm_tmem64(uint32_t d_addr, uint32_t a_addr) {
+// activation taps: a thread's packed int8 words also go to its image's row in global memory.  Nothing in the kernel reads
+// them back, so a plain generic-proxy store with a streaming hint needs no barrier.
+__device__ __forceinline__ void st_global_cs_v4(int8_t *p, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+    asm volatile("st.global.cs.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d));
+}
+
+// hidden-layer epilogue, the common 64-wide case: one TMEM load of the whole row, one TMEM store of the 16 packed words.
+// kTaps: tap (null: this row is not wanted) receives the same 16 words.
+template <bool kTaps>
+__device__ __forceinline__ void relunorm_tmem64(uint32_t d_addr, uint32_t a_addr, int8_t *tap) {
     uint32_t v[64];
     tmem_ld_x64(d_addr, v);
     tmem_ld_wait();
@@ -186,6 +198,10 @@ __device__ __forceinline__ void relunorm_tmem64(uint32_t d_addr, uint32_t a_addr
 #pragma unroll
         for (int q = 0; q < 8; q++) w[q] = norm_pack4(v[32 * h + 4 * q], v[32 * h + 4 * q + 1], v[32 * h + 4 * q + 2], v[32 * h + 4 * q + 3], k);
         tmem_st_x8(a_addr + 8 * h, w);
+        if (kTaps && tap) {
+            st_global_cs_v4(tap + 32 * h, w[0], w[1], w[2], w[3]);
+            st_global_cs_v4(tap + 32 * h + 16, w[4], w[5], w[6], w[7]);
+        }
     }
     tmem_st_wait();
 }
@@ -193,7 +209,8 @@ __device__ __forceinline__ void relunorm_tmem64(uint32_t d_addr, uint32_t a_addr
 // hidden-layer epilogue for every other width: D[tmem, n_pad columns] -> A[tmem, n_pad/4 columns] in two passes over
 // TMEM (row maximum first, then requantise), 32 columns at a time -- wide layers (Binary-160) would not fit the
 // register budget in one pass, narrow ones (16..48) do not need it.
-__device__ __forceinline__ void relunorm_tmem(uint32_t d_addr, uint32_t a_addr, uint32_t n_pad) {
+template <bool kTaps>
+__device__ __forceinline__ void relunorm_tmem(uint32_t d_addr, uint32_t a_addr, uint32_t n_pad, int8_t *tap) {
     {
         int m = 0;
         const uint32_t n32 = n_pad & ~31u;   // 32-column chunks, then at most one 16-column tail
@@ -220,6 +237,10 @@ __device__ __forceinline__ void relunorm_tmem(uint32_t d_addr, uint32_t a_addr, 
 #pragma unroll
             for (int q = 0; q < 8; q++) w[q] = norm_pack4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], k);
             tmem_st_x8(a_addr + (c >> 2), w);
+            if (kTaps && tap) {
+                st_global_cs_v4(tap + c, w[0], w[1], w[2], w[3]);
+                st_global_cs_v4(tap + c + 16, w[4], w[5], w[6], w[7]);
+            }
         }
         if (n32 < n_pad) {
             uint32_t v[16], w[4];
@@ -228,6 +249,7 @@ __device__ __forceinline__ void relunorm_tmem(uint32_t d_addr, uint32_t a_addr, 
 #pragma unroll
             for (int q = 0; q < 4; q++) w[q] = norm_pack4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], k);
             tmem_st_x4(a_addr + (n32 >> 2), w);
+            if (kTaps && tap) st_global_cs_v4(tap + n32, w[0], w[1], w[2], w[3]);
         }
     }
     tmem_st_wait();
@@ -262,7 +284,8 @@ __device__ __forceinline__ void for_chunks32_pipelined(uint32_t d_addr, uint32_t
         tmem_ld_wait();
     }
 }
-__device__ __forceinline__ void relunorm_smem(uint32_t d_addr, uint32_t a_slot_addr, uint32_t row, uint32_t n_pad) {
+template <bool kTaps>
+__device__ __forceinline__ void relunorm_smem(uint32_t d_addr, uint32_t a_slot_addr, uint32_t row, uint32_t n_pad, int8_t *tap) {
     int m = 0;
     const uint32_t n32 = n_pad & ~31u;
     for_chunks32_pipelined(d_addr, n32, [&](const uint32_t (&v)[32], uint32_t) {
@@ -283,6 +306,10 @@ __device__ __forceinline__ void relunorm_smem(uint32_t d_addr, uint32_t a_slot_a
         for (int q = 0; q < 8; q++) w[q] = norm_pack4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], k);
         st_shared_v4(a_row + c * 128, w[0], w[1], w[2], w[3]);            // K-step c / 32: block of 4096 B
         st_shared_v4(a_row + c * 128 + 128, w[4], w[5], w[6], w[7]);
+        if (kTaps && tap) {
+            st_global_cs_v4(tap + c, w[0], w[1], w[2], w[3]);
+            st_global_cs_v4(tap + c + 16, w[4], w[5], w[6], w[7]);
+        }
     });
     if (n32 < n_pad) {   // (the K-step's second chunk multiplies zero weights)
         uint32_t v[16], w[4];
@@ -291,6 +318,7 @@ __device__ __forceinline__ void relunorm_smem(uint32_t d_addr, uint32_t a_slot_a
 #pragma unroll
         for (int q = 0; q < 4; q++) w[q] = norm_pack4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], k);
         st_shared_v4(a_row + n32 * 128, w[0], w[1], w[2], w[3]);
+        if (kTaps && tap) st_global_cs_v4(tap + n32, w[0], w[1], w[2], w[3]);
     }
     fence_proxy_async_smem();   // generic-proxy writes -> visible to the tensor core's async-proxy reads
 }
@@ -360,7 +388,9 @@ __device__ __forceinline__ void issue_layer_ss(const ChainParams &P, int l, uint
 // Float input then costs 1 024 B of HBM traffic per image once, instead of 1 024 + 256 (quantise kernel) + 256 (this kernel).
 // kSmemA: wide models -- the hidden layers' activations go through shared memory instead of TMEM columns (relunorm_smem), so
 // that a tile slot is the accumulator alone and one more slot fits (Binary-160: 3 x 160 columns instead of 2 x 208).
-template <int kSlots, bool kTrace, bool kGather, bool kManyClasses, bool kFloatIn = false, bool kFourWG = false, bool kSmemA = false>
+// kTaps: the hidden layers' int8 rows are also stored to P.tap[l] (activation taps), from the registers that already hold them.
+template <int kSlots, bool kTrace, bool kGather, bool kManyClasses, bool kFloatIn = false, bool kFourWG = false, bool kSmemA = false,
+          bool kTaps = false>
 __global__ void __launch_bounds__(kFloatIn ? kFloatWG * 160 + 32 * kFloatQuantWarps : (kFourWG ? kMaxWG : kMaxWG2) * 160, 1)
 fc_chain_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_constant__ ChainParams P) {
     extern __shared__ uint8_t smem_raw[];
@@ -534,9 +564,14 @@ fc_chain_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_consta
                             if (kFloatIn) mbar_arrive(&bar_free[i % n_st]);
                             else issue_tile_load(i + n_st);
                         }
-                        if (kSmemA) relunorm_smem(d_tm, smem_base + P.off_a + (g * kSlots + q) * P.a_slot_bytes, quarter * 32 + lane, n_pad_l);
-                        else if (n_pad_l == 64) relunorm_tmem64(d_tm, d_tm + a_off);
-                        else relunorm_tmem(d_tm, d_tm + a_off, n_pad_l);
+                        int8_t *tap = nullptr;
+                        if (kTaps) {   // rows of a ragged last tile at or beyond n store nothing
+                            const size_t img = (size_t)(tile0 + i * tile_step) * kTileM + quarter * 32 + lane;
+                            if (P.tap[l] && img < P.n) tap = P.tap[l] + img * P.tap_stride[l];
+                        }
+                        if (kSmemA) relunorm_smem<kTaps>(d_tm, smem_base + P.off_a + (g * kSlots + q) * P.a_slot_bytes, quarter * 32 + lane, n_pad_l, tap);
+                        else if (n_pad_l == 64) relunorm_tmem64<kTaps>(d_tm, d_tm + a_off, tap);
+                        else relunorm_tmem<kTaps>(d_tm, d_tm + a_off, n_pad_l, tap);
                         // this thread's reads of D and writes of A are complete: tell the issuer (128 fire-and-forget arrivals per
                         // step; measured faster than syncwarp + one elected arrival: fewer instructions)
                         tc_fence_before();
@@ -797,6 +832,7 @@ FcChainPlan *fc_chain_plan_create(const FcLayerDev *layers, int n_layers, uint32
     }
     p.w_bytes = w_off;
     p.n_classes = layers[n_layers - 1].n_out;
+    for (int l = 0; l + 1 < n_layers; l++) p.tap_stride[l] = layers[l + 1].k_pad;
     p.tmem_a_off = round_up(d_cols, 32);
     p.tmem_wg_cols = p.tmem_a_off + round_up(std::max(a_cols, 1u), 16);
     if (p.tmem_wg_cols > 512) { delete plan; return fail("fused path: model does not fit the 512 TMEM columns"); }
@@ -911,7 +947,14 @@ FcChainPlan *fc_chain_plan_create(const FcLayerDev *layers, int n_layers, uint32
         cudaFuncSetAttribute(fc_chain_kernel<1, false, true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
         cudaFuncSetAttribute(fc_chain_kernel<1, false, false, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
         cudaFuncSetAttribute(fc_chain_kernel<1, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
-        cudaFuncSetAttribute(fc_chain_kernel<2, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess) {
+        cudaFuncSetAttribute(fc_chain_kernel<2, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<1, false, false, false, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<2, false, false, false, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<1, false, false, true, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<2, false, false, true, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<1, false, false, false, false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<1, false, false, true, false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess ||
+        cudaFuncSetAttribute(fc_chain_kernel<1, false, false, false, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_any) != cudaSuccess) {
         fc_chain_plan_destroy(plan);
         return fail("cannot opt in to the required dynamic shared memory");
     }
@@ -958,10 +1001,13 @@ static const CUtensorMap *plan_tensor_map(FcChainPlan *plan, const int8_t *in, s
 }
 
 int fc_chain_launch(FcChainPlan *plan, const int8_t *in, size_t n, int32_t *logits, uint32_t *labels, const GatherDst *gather,
-                    cudaStream_t st) {
+                    cudaStream_t st, const FcTaps *taps) {
     if (n == 0) return 0;
     if (n > 0x7fffff00ull) return -2;
+    if (taps && gather) return -7;
     ChainParams p = plan->p;
+    if (taps)
+        for (int l = 0; l + 1 < p.n_layers; l++) p.tap[l] = taps->act[l];
     p.logits = logits;
     p.labels = labels;
     p.n = n;
@@ -996,18 +1042,22 @@ int fc_chain_launch(FcChainPlan *plan, const int8_t *in, size_t n, int32_t *logi
     const CUtensorMap &tmap = *tmap_p;
     unsigned grid = (unsigned)std::min<uint32_t>(p.n_tiles, (uint32_t)plan->sm_count);
     long long *d_trace = nullptr;
-    const char *trace_path = (plan->trace_path.empty() || gather || plan->p.n_classes > 16 || p.n_wg > (uint32_t)kMaxWG2) ? nullptr : plan->trace_path.c_str();   // diagnostics build path
+    const char *trace_path = (plan->trace_path.empty() || gather || taps || plan->p.n_classes > 16 || p.n_wg > (uint32_t)kMaxWG2) ? nullptr : plan->trace_path.c_str();   // diagnostics build path
     if (trace_path) { cudaMalloc(&d_trace, 2048 * sizeof(long long)); cudaMemset(d_trace, 0, 2048 * sizeof(long long)); }
     p.trace = d_trace;
     // Mode 2 drops the grid-dependency wait, i.e. EVERY ordering against the work enqueued before this launch on the stream
     // (the previous bnm launch and any producer kernel of `images` alike).  The library keeps the wait whenever it can see the
     // promise being broken: first launch on this plan / another stream / a buffer of the previous launch reused.
-    bool independent = plan->overlap == 2 && plan->prev_valid && plan->prev_stream == st && in != plan->prev_in &&
+    // A taps launch is a plain launch whatever the overlap mode (its rows are a debugging aid, not a throughput path), and the
+    // launch after it is not declared independent of it.
+    const int overlap = taps ? 0 : plan->overlap;
+    bool independent = overlap == 2 && plan->prev_valid && plan->prev_stream == st && in != plan->prev_in &&
                        logits != plan->prev_logits && (labels == nullptr || labels != plan->prev_labels);
     p.wait_prior_grid = !independent;
-    p.early_trigger = plan->overlap != 0 && grid == (unsigned)plan->sm_count;
+    p.early_trigger = overlap != 0 && grid == (unsigned)plan->sm_count;
+    if (taps) p.stagger_cycles = 0;
     if (plan->stagger_override >= 0) p.stagger_cycles = (uint32_t)plan->stagger_override;
-    plan->prev_in = in; plan->prev_logits = logits; plan->prev_labels = labels; plan->prev_stream = st; plan->prev_valid = true;
+    plan->prev_in = in; plan->prev_logits = logits; plan->prev_labels = labels; plan->prev_stream = st; plan->prev_valid = !taps;
     if (trace_path) {
         if (p.n_slots == 1) fc_chain_kernel<1, true, false, false><<<grid, plan->threads, plan->smem_bytes, st>>>(tmap, p);
         else fc_chain_kernel<2, true, false, false><<<grid, plan->threads, plan->smem_bytes, st>>>(tmap, p);
@@ -1022,7 +1072,7 @@ int fc_chain_launch(FcChainPlan *plan, const int8_t *in, size_t n, int32_t *logi
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
-        cfg.numAttrs = plan->overlap ? 1 : 0;
+        cfg.numAttrs = overlap ? 1 : 0;
         const bool g = p.n_lab_dst || p.n_log_dst;
         const bool many = p.n_classes > 16;
         const bool smem_a = !g && !many && plan->sa_smem_bytes != 0;
@@ -1036,12 +1086,19 @@ int fc_chain_launch(FcChainPlan *plan, const int8_t *in, size_t n, int32_t *logi
         cudaError_t e;
 #define BNM_LAUNCH(S, G, M) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<S, false, G, M>, tmap, p)
 #define BNM_LAUNCH4(G, M) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<1, false, G, M, false, true>, tmap, p)
-        if (smem_a) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<1, false, false, false, false, false, true>, tmap, p);
+#define BNM_LAUNCH_T(S, M, W4) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<S, false, false, M, false, W4, false, true>, tmap, p)
+        if (taps) {
+            if (smem_a) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<1, false, false, false, false, false, true, true>, tmap, p);
+            else if (p.n_wg > (uint32_t)kMaxWG2) { if (many) BNM_LAUNCH_T(1, true, true); else BNM_LAUNCH_T(1, false, true); }
+            else if (p.n_slots == 1) { if (many) BNM_LAUNCH_T(1, true, false); else BNM_LAUNCH_T(1, false, false); }
+            else { if (many) BNM_LAUNCH_T(2, true, false); else BNM_LAUNCH_T(2, false, false); }
+        } else if (smem_a) e = cudaLaunchKernelEx(&cfg, fc_chain_kernel<1, false, false, false, false, false, true>, tmap, p);
         else if (p.n_wg > (uint32_t)kMaxWG2) { if (g) { if (many) BNM_LAUNCH4(true, true); else BNM_LAUNCH4(true, false); } else { if (many) BNM_LAUNCH4(false, true); else BNM_LAUNCH4(false, false); } }
         else if (p.n_slots == 1) { if (g) { if (many) BNM_LAUNCH(1, true, true); else BNM_LAUNCH(1, true, false); } else { if (many) BNM_LAUNCH(1, false, true); else BNM_LAUNCH(1, false, false); } }
         else { if (g) { if (many) BNM_LAUNCH(2, true, true); else BNM_LAUNCH(2, true, false); } else { if (many) BNM_LAUNCH(2, false, true); else BNM_LAUNCH(2, false, false); } }
 #undef BNM_LAUNCH
 #undef BNM_LAUNCH4
+#undef BNM_LAUNCH_T
         if (e != cudaSuccess) return -4;
     }
     if (trace_path) {   // diagnostics only: synchronous dump of the phase clocks

@@ -79,10 +79,14 @@ FcChainPlan *fc_chain_plan_create(const FcLayerDev *layers, int n_layers, uint32
 void fc_chain_plan_destroy(FcChainPlan *p);
 // 0 plain launches, 1 programmatic dependent launch (inputs read after the previous kernel completed), 2 launches declared independent
 void fc_chain_plan_set_overlap(FcChainPlan *p, int mode);
+// activation taps of the fused chain: act[l] = int8 [n][k_pad of layer l + 1] receiving hidden layer l's ReLUNorm rows (null: not
+// wanted; bytes past the layer's n_pad are not written), l < n_layers - 1
+struct FcTaps { int8_t *act[kMaxFcLayers]; };
 // images int8 [n][in_bytes] (device, 16B aligned) -> logits int32 [n][n_classes], labels uint32 [n] (may be null)
 // gather (may be null): extra destination buffers every row is also stored to (peer memory), fused into the epilogue
+// taps (may be null; not with gather): a plain launch (mode 0) that also stores the hidden layers' rows
 int fc_chain_launch(FcChainPlan *p, const int8_t *in, size_t n, int32_t *logits, uint32_t *labels, const GatherDst *gather,
-                    cudaStream_t st);
+                    cudaStream_t st, const FcTaps *taps = nullptr);
 
 // float32 images [n][in_bytes] (elements) -> logits / labels with the input scaling of test_inference.py:140-141 fused into the
 // kernel's load stage; supported for image rows of up to 256 elements and up to 16 classes

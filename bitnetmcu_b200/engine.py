@@ -13,7 +13,7 @@ torch is used only as plumbing for device memory / streams in ``infer_device``.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -103,6 +103,59 @@ class Engine:
         _lib.check(self.lib.bnm_infer_batch_device(self.handle, C.c_void_p(images.data_ptr()), n, C.c_void_p(logits.data_ptr()),
                                                    lab_ptr, C.c_void_p(stream)), "bnm_infer_batch_device")
 
+
+    # ---- activation taps: the int8 rows between the layers (include/bitnetmcu_b200.h section 7) -------------
+    @property
+    def n_taps(self) -> int:
+        """Taps of this model: one per hidden FC layer, plus the CNN features (tap 0) for CNN models."""
+        return int(self.lib.bnm_model_n_taps(self.handle))
+
+    def tap_shapes(self) -> List[Tuple[int, int]]:
+        """(width, stride) per tap: real int8 values per row, and bytes between rows of a tap buffer."""
+        return [(int(self.lib.bnm_model_tap_width(self.handle, t)), int(self.lib.bnm_model_tap_stride(self.handle, t)))
+                for t in range(self.n_taps)]
+
+    def infer_taps(self, images: np.ndarray) -> Tuple[np.ndarray, np.ndarray, List[np.ndarray]]:
+        """As ``infer``, plus every tap: (logits int32 [n, n_classes], labels uint32 [n], [int8 [n, width] per tap])."""
+        imgs = np.ascontiguousarray(images, dtype=np.int8).reshape(-1, self.img_bytes)
+        n = imgs.shape[0]
+        logits = np.empty((n, self.n_classes), dtype=np.int32)
+        labels = np.empty(n, dtype=np.uint32)
+        bufs = [np.empty((n, stride), dtype=np.int8) for _, stride in self.tap_shapes()]
+        taps = _lib.BnmTaps()
+        for t, b in enumerate(bufs):
+            taps.act[t] = b.ctypes.data
+        _lib.check(self.lib.bnm_infer_batch_taps(self.handle, _ptr(imgs), n, _ptr(logits), _ptr(labels), C.byref(taps)),
+                   "bnm_infer_batch_taps")
+        return logits, labels, [b[:, :w] for b, (w, _) in zip(bufs, self.tap_shapes())]
+
+    def infer_device_taps(self, images, logits, labels, taps: Sequence, stream: Optional[int] = None) -> None:
+        """As ``infer_device``, plus the taps: ``taps[t]`` is a torch.int8 [n, stride of t] tensor on this GPU, or None when tap t
+        is not wanted.  Only int8 images: float input has no taps."""
+        import torch
+        n = images.shape[0]
+        if images.dtype != torch.int8:
+            raise _lib.BnmError(f"activation taps need int8 images (got {images.dtype}): float input has no taps")
+        if stream is None:
+            stream = torch.cuda.current_stream(images.device).cuda_stream
+        assert images.is_contiguous() and logits.is_contiguous() and logits.dtype == torch.int32
+        assert images.shape[1] == self.img_bytes and tuple(logits.shape) == (n, self.n_classes)
+        assert len(taps) <= _lib.MAX_TAPS
+        lab_ptr = None
+        if labels is not None:
+            assert labels.is_contiguous() and labels.element_size() == 4 and labels.numel() == n
+            lab_ptr = C.c_void_p(labels.data_ptr())
+        shapes = self.tap_shapes()
+        tt = _lib.BnmTaps()
+        for t, b in enumerate(taps):
+            if b is None:
+                continue
+            assert t < len(shapes), f"tap {t}: the model has {len(shapes)} taps"
+            assert b.dtype == torch.int8 and b.is_contiguous() and tuple(b.shape) == (n, shapes[t][1]), \
+                f"tap {t}: want a contiguous torch.int8 [{n}, {shapes[t][1]}] tensor"
+            tt.act[t] = b.data_ptr()
+        _lib.check(self.lib.bnm_infer_batch_device_taps(self.handle, C.c_void_p(images.data_ptr()), n, C.c_void_p(logits.data_ptr()),
+                                                        lab_ptr, C.byref(tt), C.c_void_p(stream)), "bnm_infer_batch_device_taps")
 
     def inference_quantized(self, input_data: np.ndarray) -> np.ndarray:
         """``QuantizedModel.inference_quantized`` (/root/reference/BitNetMCU.py:420-535) on the GPU: float32 images [n, img_bytes]

@@ -22,7 +22,7 @@ from __future__ import annotations
 import re
 import struct
 from dataclasses import dataclass, field
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
@@ -117,6 +117,17 @@ class Model:
             o1, o2, o3 = (xy - 2) ** 2, (xy - 4) ** 2, ((xy - 4) // 2 - 2) ** 2
             macs += self.channels * 9 * (o1 + o2 + o3)
         return macs
+
+    def tap_shapes(self) -> List[Tuple[int, int]]:
+        """(width, stride) of every activation tap (include/bitnetmcu_b200.h section 7), from the layer table alone: the CNN
+        features (C*4 values, rows of round_up(C*4, 16) bytes) for CNN models, then per hidden FC layer its n_out values in rows
+        of round_up(n_in of the next layer, 32) bytes."""
+        fc = self.fc_layers
+        shapes = []
+        if self.model_class == MODEL_CNNMNIST:
+            shapes.append((self.channels * 4, -(-self.channels * 4 // 16) * 16))
+        shapes += [(fc[l].n_out, -(-fc[l + 1].n_in // 32) * 32) for l in range(len(fc) - 1)]
+        return shapes
 
     def describe(self) -> str:
         parts = []

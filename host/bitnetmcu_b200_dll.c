@@ -61,3 +61,10 @@ EXPORT int InferenceBatch(const int8_t *images, size_t n, int32_t *logits, uint3
 
 EXPORT uint32_t InferenceNumClasses(void) { return BNM_MODEL_N_CLASSES; }
 EXPORT const char *InferenceLastError(void) { return bnm_last_error(); }
+
+/* dll.c:29-37: one activation row as the firmware's UART dump prints it -- "%d, " per value, a line break after every 16 */
+EXPORT void printactivations(uint8_t *activations, int32_t n_activations)
+{
+    for (int32_t i = 0; i < n_activations; i++)
+        printf((i % 16 == 15) ? "%d, \n" : "%d, ", activations[i]);
+}

@@ -212,6 +212,36 @@ BNM_API int bnm_quantize_images_device(const float *images, size_t n, uint32_t e
  * ------------------------------------------------------------------------------------------- */
 BNM_API int bnm_emulate_inference_quantized(bnm_model *m, const float *images, size_t n, double *logits);
 
+/* ---------------------------------------------------------------------------------------------
+ * 7. Activation taps: the int8 rows between the layers (what the reference's printactivations() dumps, dll.c:29-37,102-109)
+ *
+ *    A tap is the int8 row that a ReLUNorm of BitMnistInference writes into layer_in and the next layer then reads.  Taps are
+ *    numbered in chain order: for CNN models tap 0 is the C*4 features after the front-end's ReLUNorm (dll.c:80; channel-major,
+ *    four pooled values per channel); then, for both model classes, one tap per hidden FC layer (every FC layer but the last,
+ *    whose normalised row the reference never uses).  An FC model with L layers has L-1 taps, a CNN model L; at most 8.
+ *    Tap t has
+ *      width   real values: C*4 for the CNN features, the producing layer's n_out for a hidden FC row;
+ *      stride  bytes between rows: round_up(C*4, 16) for the CNN features, round_up(n_in of the next layer, 32) for a hidden FC
+ *              row (Ternary layers pad n_in to a multiple of 10: a 64-wide hidden row of a ternary chain has stride 96).
+ *    Bytes between width and stride are unspecified (the next layer multiplies them by zero weights).
+ *
+ *    The _taps calls compute exactly what bnm_infer_batch[_device] computes (bit-identical logits and labels) and also store
+ *    every requested tap: act[t] = int8 [n][stride of t], 16-byte aligned, or NULL when tap t is not wanted; taps == NULL or all
+ *    entries NULL is the plain call.  Not for float input or the fused gather (BNM_E_UNSUPPORTED).  A taps launch is a plain
+ *    launch (ordinary stream semantics) whatever BNM_OPT_LAUNCH_OVERLAP says: a debugging path, not a throughput path.
+ * ------------------------------------------------------------------------------------------- */
+#define BNM_MAX_TAPS 8
+typedef struct bnm_taps { int8_t *act[BNM_MAX_TAPS]; } bnm_taps;   /* NULL entry = tap not wanted */
+BNM_API uint32_t bnm_model_n_taps(const bnm_model *m);
+BNM_API uint32_t bnm_model_tap_width(const bnm_model *m, uint32_t t);    /* 0 when t >= n_taps */
+BNM_API uint32_t bnm_model_tap_stride(const bnm_model *m, uint32_t t);   /* 0 when t >= n_taps */
+/* device buffers on the model's GPU, asynchronous on `stream` (as bnm_infer_batch_device) */
+BNM_API int bnm_infer_batch_device_taps(bnm_model *m, const int8_t *images, size_t n, int32_t *logits, uint32_t *labels,
+                                        const bnm_taps *taps, void *stream);
+/* host buffers (as bnm_infer_batch; tap rows at the same strides), one stream, chunks of BNM_OPT_CHUNK_IMAGES images */
+BNM_API int bnm_infer_batch_taps(bnm_model *m, const int8_t *images, size_t n, int32_t *logits, uint32_t *labels,
+                                 const bnm_taps *taps);
+
 #ifdef __cplusplus
 }
 #endif
